@@ -8,10 +8,13 @@ Contract (driver):  python bench.py --gpus N --steps K --warmup W [--impl refere
     runs its own sequence (seed = rank) — weak scaling, no collective on the data path, poses gathered at the end.
   * before the W warm-up steps each pipeline is PRIMED with --prime scans (setup, untimed) so the timed region
     sees a steady-state local map instead of an almost empty one.
-  * a timed WINDOW is exactly K consecutive scans of the stream, bracketed by barrier + synchronize and timed with
-    CUDA events on the launching stream. The stream simply continues for --repeats R windows (R*K scans in all);
-    every number in the line is the MEDIAN window (per rank), then the max over ranks; min/max and the per-rank
-    medians are in `windows`. (One 20-scan window is ~3 ms: a single host hiccup used to move the result by 2x.)
+  * every timed leg times exactly K consecutive scans of the stream, split into --repeats R consecutive WINDOWS (default
+    one per 20 scans), each bracketed by barrier + synchronize and timed with CUDA events on the launching stream;
+    every number in the line comes from the MEDIAN window time per scan (per rank), then the max over ranks; min/max and
+    the per-rank medians are in `windows`. (One 20-scan window is ~3 ms: a single host hiccup used to move the result by 2x.)
+  * --dump-outputs DIR: after the timed scans, rank 0 writes what the last timed scan returned to its caller as float64
+    .npy files (pose.npy, preprocessed.npy, source.npy); the inputs depend only on the arguments, so two builds can be
+    compared output for output.
   * value  = scans/s with the scans already resident in HBM, frames queued (kb_pipeline_register_frames, device layout)
   * e2e    = scans/s through the host-facing C-ABI call with pinned HOST buffers: H2D of every scan and D2H of every
              result inside the timed region (kb_pipeline_register_frames, host layout); `blocking_calls` is the same
@@ -47,9 +50,10 @@ WORKLOADS = {
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20, help="scans per timed window")
+    ap.add_argument("--steps", type=int, default=20, help="timed scans of every timed leg")
     ap.add_argument("--warmup", type=int, default=5)
-    ap.add_argument("--repeats", type=int, default=9, help="timed windows of --steps scans each (the stream continues); medians are reported")
+    ap.add_argument("--repeats", type=int, default=None,
+                    help="timing windows the --steps scans are split into (default: one per 20 scans); medians are reported")
     ap.add_argument("--prime", type=int, default=100, help="scans registered before warm-up (steady-state map)")
     ap.add_argument("--workload", default="kitti", choices=sorted(WORKLOADS))
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
@@ -59,7 +63,18 @@ def parse():
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-extra", action="store_true", help="skip the f32 / profile / trajectory side legs")
     ap.add_argument("--no-clocks", action="store_true", help="diagnostic: do not sample clocks (an invalid run by the bench contract)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed scans, write what the last one returned (pose, preprocessed frame, source points) as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1 or (args.repeats is not None and args.repeats < 1):
+        ap.error("--steps and --repeats must be at least 1")
+    return args
+
+
+def window_sizes(args):
+    """the --steps timed scans split into consecutive windows whose sizes differ by at most one"""
+    R = min(args.steps, args.repeats or max(1, args.steps // 20))
+    return [args.steps // R + (r < args.steps % R) for r in range(R)]
 
 
 def make_lidar(workload, seed, device):
@@ -80,8 +95,8 @@ def oracle_kwargs(workload):
 def common_config(args, world):
     """identical in both arms (the driver compares the two dicts)"""
     return {"workload": WORKLOADS[args.workload]["name"], "prime_scans": args.prime, "sequences": world,
-            "windows": args.repeats, "steps_per_window": args.steps,
-            "statistic": "median over the windows of the per-window scans/s (each window = exactly --steps consecutive scans); max over ranks of the per-rank median time",
+            "timed_steps": args.steps, "windows": len(window_sizes(args)),
+            "statistic": "median over the windows of the per-window time per scan (the --steps timed scans split into consecutive windows); max over ranks of the per-rank median time",
             "l2": "every step consumes a new scan (1.5 MB KITTI / 3 MB Ouster); the local map (the state of the stream) is legitimately L2-resident across steps"}
 
 
@@ -204,7 +219,7 @@ def thread_candidates():
 def run_reference(args, rank, world):
     """the reference's CPU implementation of the path on the host cores (oracle port). At --gpus N the job is
     N independent sequences (one per GPU in our arm): here they run concurrently on the host, each with its
-    share of the cores. Same windows as our arm: R windows of K scans, value = N * K / median window time."""
+    share of the cores. Same windows as our arm: K scans in R windows, value = N / median window time per scan."""
     if rank != 0:
         return
     from concurrent.futures import ThreadPoolExecutor
@@ -212,9 +227,11 @@ def run_reference(args, rank, world):
     import torch
     dev = "cuda" if torch.cuda.is_available() else "cpu"
     nseq = max(1, args.gpus)
-    R = max(1, min(args.repeats, 5))  # bounded: the whole run must end within a few minutes on a slow host
+    sizes = window_sizes(args)
+    starts = np.cumsum([0] + sizes)
+    R = len(sizes)
     head = args.prime + args.warmup
-    n_total = head + R * args.steps
+    n_total = head + args.steps
     kw = oracle_kwargs(args.workload)
     streams = []
     for sid in range(nseq):
@@ -234,20 +251,20 @@ def run_reference(args, rank, world):
         list(ex.map(lambda sid: run(sid, 0, head), range(nseq)))
         for r in range(R):
             t0 = time.perf_counter()
-            list(ex.map(lambda sid: run(sid, head + r * args.steps, head + (r + 1) * args.steps), range(nseq)))
+            list(ex.map(lambda sid: run(sid, head + starts[r], head + starts[r + 1]), range(nseq)))
             win.append(time.perf_counter() - t0)
-    dt = float(np.median(win))
-    val = nseq * args.steps / dt
+    dt = float(np.median(np.array(win) / sizes))  # seconds per scan
+    val = nseq / dt
     cfg = common_config(args, nseq)
     line = {"impl": "reference", "metric": WORKLOADS[args.workload]["metric"], "value": val, "unit": "scans/s", "n_gpus": args.gpus,
-            "steps": args.steps, "warmup": args.warmup, "ms_per_step": dt / args.steps * 1e3,
+            "steps": args.steps, "warmup": args.warmup, "ms_per_step": dt * 1e3,
             "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f64", "data": "synthetic",
             "config": cfg,
-            "windows": {"ms": [w * 1e3 for w in win], "timed": R, "note": "the reference arm times at most 5 of the --repeats windows (bounded run time)"},
+            "windows": {"ms": [w * 1e3 for w in win], "scans": sizes},
             "note": "reference CPU path = dependency-free restatement of cpp/kiss_icp (oracle port, OpenMP for TBB); the real "
                     "TBB/Eigen build needs network-fetched deps. N sequences run concurrently on the host cores.",
             "cpu_baseline": {"value": val, "unit": "scans/s", "cores": nt * nseq, "kind": "port",
-                             "sample": f"{nseq} x {R} windows of {args.steps} scans after {head} untimed; {nt} OpenMP "
+                             "sample": f"{nseq} x {args.steps} scans in {R} windows after {head} untimed; {nt} OpenMP "
                                        f"threads per sequence (fastest single-sequence count of {thread_candidates()} "
                                        f"capped at cpus/sequences) on {ncpu} cpus"},
             "e2e": {"value": val, "unit": "scans/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}}
@@ -286,9 +303,10 @@ def main():
 
     seq = sharding.sequences_of_rank(rank, world, world)[0]
     lidar = make_lidar(args.workload, seq, dev)
-    Kw, R = args.steps, max(1, args.repeats)
+    Kw, sizes = args.steps, window_sizes(args)
+    starts, R = np.cumsum([0] + sizes), len(sizes)
     head = args.prime + args.warmup
-    n_total = head + R * Kw
+    n_total = head + Kw
     scans_dev = []
     for k in range(n_total):
         p, t = lidar.scan_torch(k)
@@ -341,13 +359,13 @@ def main():
         return e0.elapsed_time(e1)
 
     def timed_windows(fn_of_window):
-        """R windows of K scans each -> (this rank's window times [ms], median over windows maxed over ranks)"""
+        """K scans in R windows -> (this rank's window times [ms], K x the median window time per scan, maxed over ranks)"""
         ms = [window(lambda r=r: fn_of_window(r)) for r in range(R)]
-        return ms, sharding.max_over_ranks(float(np.median(ms)), dev)
+        return ms, sharding.max_over_ranks(float(np.median(np.array(ms) / sizes)) * Kw, dev)
 
     def win_scans(pool, r):
         off = head if len(pool) == n_total else 0  # pools hold either the whole stream or only the timed part
-        return pool[off + r * Kw: off + (r + 1) * Kw]
+        return pool[off + starts[r]: off + starts[r + 1]]
 
     warm = scans_dev[args.prime:head]
     legs = {}
@@ -360,10 +378,13 @@ def main():
     if rank == 0:
         sampler.mark()
     l0 = launches(icp)
-    legs["value"] = timed_windows(lambda r: queued(icp, win_scans(scans_dev, r), 2))
-    gpu_launches = (launches(icp) - l0) // R
+    value_poses = []
+    legs["value"] = timed_windows(lambda r: value_poses.append(queued(icp, win_scans(scans_dev, r), 2)))
+    gpu_launches = launches(icp) - l0
     ms_value = legs["value"][1]
     value = world * Kw / (ms_value * 1e-3)
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, L, icp, value_poses[-1][-1])
 
     # ---------------- the same with one blocking RegisterFrame call per scan (the reference's call shape)
     icp_b = primed(head)
@@ -404,9 +425,9 @@ def main():
     same = bool(np.array_equal(icp.last_pose, icp2.last_pose) and np.array_equal(icp_b.last_pose, icp2b.last_pose)
                 and np.array_equal(icp.last_pose, icp_b.last_pose) and np.array_equal(e2e_last[-1], icp2.last_pose))
 
-    # ---------------- profiling pass (untimed): one window once more with the in-kernel phase timestamps ON
+    # ---------------- profiling pass (untimed): the timed scans once more with the in-kernel phase timestamps ON
     # (they cost ~1 us each on the kernel's critical path, so the timed passes above run without them)
-    prof_n = Kw * min(R, 3)
+    prof_n = Kw
     prof = np.zeros((prof_n, 6))
     iters = np.zeros(prof_n)
     work = np.zeros((prof_n, 2))
@@ -435,7 +456,7 @@ def main():
                "note": "register_frames, float32 host frames (native KITTI/ROS payload), widened on the device"}
     # ---------------- the reference's Python call structure (python/kiss_icp/kiss_icp.py:43-75): six module calls per scan,
     # each copying its clouds in and out (KissICP(fused=False) = preprocess, voxelize x2, threshold, align, update on the
-    # per-module C-ABI); host wall clock on rank 0, one window
+    # per-module C-ABI); host wall clock on rank 0, the K timed scans in one go
     modular = None
     if rank == 0 and world == 1 and not args.no_extra:
         try:
@@ -472,10 +493,10 @@ def main():
         return
 
     def win_summary(name):
-        a = per_rank[name]
+        a = per_rank[name] / sizes  # ms per scan of every window
         med = np.median(a, axis=1)
-        return {"median_ms_per_rank": [float(x) for x in med], "min_ms": float(a.min()), "max_ms": float(a.max()),
-                "slowest_rank": int(np.argmax(med)), "scans_per_s": world * Kw / (float(med.max()) * 1e-3)}
+        return {"scans": sizes, "median_ms_per_scan_per_rank": [float(x) for x in med], "min_ms_per_scan": float(a.min()),
+                "max_ms_per_scan": float(a.max()), "slowest_rank": int(np.argmax(med)), "scans_per_s": world / (float(med.max()) * 1e-3)}
 
     # ---------------- roofline of the dominant kernel (k_register_frame, one launch per scan)
     peaks_path = os.path.join(ROOT, "MEASURED_PEAKS.json")
@@ -547,7 +568,7 @@ def multi_stream_leg(args, K, N, L, torch, dev, S, cfg):
     sized to 1/S of the SMs (SURVEY.md 8f rank 1). Reported beside the single-stream headline, never instead."""
     import threading
     sms = torch.cuda.get_device_properties(dev).multi_processor_count
-    steps = args.steps * min(args.repeats, 3)
+    steps = args.steps
     n_total = min(args.prime, 40) + steps
     data = []
     for sid in range(S):
@@ -598,6 +619,19 @@ def multi_stream_leg(args, K, N, L, torch, dev, S, cfg):
             "ms_per_scan_per_stream": float(np.mean(walls)) / steps * 1e3,
             "note": "aggregate over S concurrent sequences on one GPU (S pipelines on S streams, each launch on 1/S of the SMs), "
                     "inputs resident in HBM, frames queued, host wall clock"}
+
+
+def dump_outputs(out_dir, L, icp, pose):
+    """what the last timed scan returned to its caller: its pose (from kb_pipeline_register_frames) and the two clouds
+    RegisterFrame returns with it (preprocessed frame, source points), all float64, ~1.6 MB per KITTI-shape scan"""
+    from kiss_icp_b200 import _native as N
+    n_pre, n_src = N.sz(0), N.sz(0)
+    N.check(L.kb_pipeline_last_cloud_sizes(icp._h, C.byref(n_pre), C.byref(n_src)))
+    pre, src = np.empty((n_pre.value, 3)), np.empty((n_src.value, 3))
+    N.check(L.kb_pipeline_last_clouds(icp._h, N.ptr(pre), n_pre.value, N.ptr(src), n_src.value))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in (("pose", np.asarray(pose, dtype=np.float64)), ("preprocessed", pre), ("source", src)):
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def profiled_traffic(tag):
@@ -706,7 +740,7 @@ def cpu_leg(args, lidar):
     thread count and the 1-thread figure (SURVEY.md 8d)."""
     from oracle import oracle as O
     kw = oracle_kwargs(args.workload)
-    n = min(args.cpu_sample, args.steps * args.repeats)
+    n = min(args.cpu_sample, args.steps)
     scans = [lidar.scan(k) for k in range(args.prime + n)]
     nt = best_thread_count(O, scans, thread_candidates(), **kw)
     icp = O.KissICP(max_num_threads=nt, **kw)

@@ -81,42 +81,47 @@ def test_host_only_parts_and_errors_without_a_gpu(mod):
             mod._voxel_down_sample(np.zeros((3, 3)), 0.5)
 
 
-REF = "/root/reference/python"
+# the python/ directory of an upstream kiss-icp checkout; its sources are not part of this repository
+REF = os.environ.get("KISS_ICP_UPSTREAM_PYTHON", "")
+HAVE_REF = bool(REF) and os.path.isdir(os.path.join(REF, "kiss_icp"))
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "kiss_icp")), reason="reference checkout not available on this machine")
 def test_reference_python_layer_imports_on_top_of_it(mod):
-    """python/kiss_icp/*.py, unmodified, with `kiss_icp.pybind.kiss_icp_pybind` supplied by this module"""
-    saved = {k: v for k, v in sys.modules.items() if k == "kiss_icp" or k.startswith("kiss_icp.")}
-    sys.path.insert(0, REF)
-    try:
-        import kiss_icp
-        pkg = types.ModuleType("kiss_icp.pybind")
-        pkg.__path__ = []
-        pkg.kiss_icp_pybind = mod
-        sys.modules["kiss_icp.pybind"] = pkg
-        sys.modules["kiss_icp.pybind.kiss_icp_pybind"] = mod
-        kiss_icp.pybind = pkg
-        import kiss_icp.mapping, kiss_icp.metrics, kiss_icp.preprocess, kiss_icp.registration, kiss_icp.voxelization  # noqa: E401,F401
-        from kiss_icp.config import load_config
-        from kiss_icp.threshold import get_threshold_estimator
-        cfg = load_config(None)
-        est = get_threshold_estimator(cfg)
-        assert est.get_threshold() == cfg.adaptive_threshold.initial_threshold
-        est.update_model_deviation(np.eye(4))
-        g = np.tile(np.eye(4), (300, 1, 1))
-        g[:, 0, 3] = np.arange(300)
-        assert max(kiss_icp.metrics.sequence_error(g, g)) < 1e-6
-        from kiss_icp_b200 import _native as N
-        from kiss_icp.kiss_icp import KissICP
-        if N.lib().kb_device_count() < 1:
-            with pytest.raises(RuntimeError, match="no CUDA device"):
-                KissICP(cfg)
-    finally:
-        sys.path.remove(REF)
-        for k in [k for k in sys.modules if k == "kiss_icp" or k.startswith("kiss_icp.")]:
-            del sys.modules[k]
-        sys.modules.update(saved)
+    """python/kiss_icp/*.py, unmodified, with `kiss_icp.pybind.kiss_icp_pybind` supplied by this module: the calls the
+    upstream layer made into it (import, default config, threshold estimate and update, KITTI metrics, KissICP's
+    constructor), recorded by tests/golden/make_pybind_calls.py, are replayed; each must be accepted and give the
+    recorded result, and without a device the pipeline's constructor must fail as it did then"""
+    import json
+    from kiss_icp_b200 import _native as N
+    golden = os.path.join(ROOT, "tests", "golden", "pybind_calls_v1")
+    log = json.load(open(golden + ".json"))
+    arrays = np.load(golden + ".npz")
+    objs = {}
+
+    def dec(v):
+        if isinstance(v, dict):
+            return objs[v["obj"]] if "obj" in v else arrays[v["array"]]
+        return [dec(x) for x in v] if isinstance(v, list) else v
+
+    assert log["meta"]["first_threshold"] == log["meta"]["initial_threshold"]
+    no_device = N.lib().kb_device_count() < 1
+    for c in log["calls"]:
+        fn = getattr(mod, c["func"]) if "func" in c else getattr(objs[c["obj"]], c["method"])
+        args, kwargs = [dec(a) for a in c["args"]], {k: dec(v) for k, v in c["kwargs"].items()}
+        if "raised" in c:
+            assert c["raised"]["type"] == "RuntimeError" and "no CUDA device" in c["raised"]["message"]
+            if no_device:
+                with pytest.raises(RuntimeError, match="no CUDA device"):
+                    fn(*args, **kwargs)
+            continue
+        r = fn(*args, **kwargs)
+        want = c["result"]
+        if isinstance(want, dict) and "obj" in want:
+            objs[want["obj"]] = r
+        elif want is None:
+            assert r is None
+        else:
+            assert np.allclose(np.asarray(r, dtype=np.float64), np.asarray(dec(want), dtype=np.float64), rtol=1e-12, atol=1e-9), (c, r)
 
 
 @pytest.mark.gpu
@@ -164,8 +169,8 @@ def test_every_bound_call_equals_the_ctypes_mirror(mod):
 
 
 class _ReferenceKissICP:
-    """python/kiss_icp/kiss_icp.py:33-80 (class KissICP) restated on the bound module — the GPU box has no reference
-    checkout; where /root/reference exists the test below uses the reference's own class instead"""
+    """python/kiss_icp/kiss_icp.py:33-80 (class KissICP) restated on the bound module; where KISS_ICP_UPSTREAM_PYTHON
+    points at an upstream checkout the test below uses the reference's own class instead"""
 
     def __init__(self, mod, max_range=100.0, voxel_size=1.0):
         self.m = mod
@@ -202,7 +207,7 @@ def test_reference_python_register_frame_loop_on_the_gpu(mod, O):
     L = synthetic.small_shape(seed=11, beams=32, cols=512, stamps="column")
     icp = None
     saved = {k: v for k, v in sys.modules.items() if k == "kiss_icp" or k.startswith("kiss_icp.")}
-    use_ref = os.path.isdir(os.path.join(REF, "kiss_icp"))
+    use_ref = HAVE_REF
     try:
         if use_ref:
             sys.path.insert(0, REF)

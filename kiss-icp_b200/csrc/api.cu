@@ -271,7 +271,7 @@ int watchdog_check(int device) {
     h[0] = 0;
     unsigned zero = 0;
     cudaMemcpyToSymbol(g_kb_wd, &zero, sizeof(zero));  // re-arm
-    static const char *names[] = {"?", "grid barrier", "ICP gather", "ICP result record", "ICP team gather", "NN bulk copy"};
+    static const char *names[] = {"?", "grid barrier", "ICP gather", "ICP result record", "ICP team gather"};
     // where every CTA of the last k_register_frame was (the launch has ended: a plain copy)
     std::string marks;
     unsigned m[256];
@@ -286,7 +286,7 @@ int watchdog_check(int device) {
     cudaGetLastError();
     return fail(KB_ERR_CUDA, "device watchdog: a kernel gave up waiting at the %s (block %u, thread %u, a=%u, b=%u; grid barrier: a = target, b = counter); "
                              "the results of that launch are invalid%s",
-                names[code < 6 ? code : 0], block, thread, a, b, marks.c_str());
+                names[code < sizeof(names) / sizeof(names[0]) ? code : 0], block, thread, a, b, marks.c_str());
 }
 
 bool g_stuck[64];
@@ -890,34 +890,13 @@ static int nn_launch(kb_map *map, const double *d_q, size_t n, double *d_p, doub
     if (n == 0) return KB_OK;
     int sms = 148;
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, map->ex->device);
-    // default: the register-staged kernel (never slower in same-box A/Bs: 1.580 vs 1.585 ms, 1.588 vs 1.695 ms);
-    // KB_NN_KERNEL=bulk selects the variant that stages the candidate blocks with cp.async.bulk + mbarrier
-    // (needs 16-byte aligned blocks: an even max_points_per_voxel <= 32; read per call)
-    const char *env = std::getenv("KB_NN_KERNEL");
-    const bool want_bulk = env && std::strcmp(env, "bulk") == 0;
-    const bool bulk = want_bulk && map->cap <= static_cast<unsigned>(NN_FLAT_CAP) && (map->cap & 1u) == 0;
     const int threads = 256;
     const size_t want = (n * 32 + threads - 1) / threads;
-    if (bulk) {
-        const size_t smem = static_cast<size_t>(NNB_WARPS) * NNB_BUF;
-        const void *k0 = reinterpret_cast<const void *>(&k_nn_query_bulk<false>), *k1 = reinterpret_cast<const void *>(&k_nn_query_bulk<true>);
-        for (const void *k : {k0, k1})
-            if (std::find(map->ex->smem_opted.begin(), map->ex->smem_opted.end(), k) == map->ex->smem_opted.end()) {
-                CK(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
-                map->ex->smem_opted.push_back(k);
-            }
-        const unsigned blocks = static_cast<unsigned>(std::min<size_t>(want, static_cast<size_t>(sms) * 3));  // 3 CTAs/SM, grid-stride
-        if (d_cand)
-            k_nn_query_bulk<true><<<blocks, threads, smem, map->ex->stream>>>(map->view(), d_q, n, d_p, d_d, d_cand);
-        else
-            k_nn_query_bulk<false><<<blocks, threads, smem, map->ex->stream>>>(map->view(), d_q, n, d_p, d_d, nullptr);
-    } else {
-        const unsigned blocks = static_cast<unsigned>(std::min<size_t>(want, static_cast<size_t>(sms) * 4));  // 4 CTAs/SM, grid-stride
-        if (d_cand)
-            k_nn_query<true><<<blocks, threads, 0, map->ex->stream>>>(map->view(), d_q, n, d_p, d_d, d_cand);
-        else
-            k_nn_query<false><<<blocks, threads, 0, map->ex->stream>>>(map->view(), d_q, n, d_p, d_d, nullptr);
-    }
+    const unsigned blocks = static_cast<unsigned>(std::min<size_t>(want, static_cast<size_t>(sms) * 4));  // 4 CTAs/SM, grid-stride
+    if (d_cand)
+        k_nn_query<true><<<blocks, threads, 0, map->ex->stream>>>(map->view(), d_q, n, d_p, d_d, d_cand);
+    else
+        k_nn_query<false><<<blocks, threads, 0, map->ex->stream>>>(map->view(), d_q, n, d_p, d_d, nullptr);
     ++map->ex->launches;
     CK(cudaGetLastError());
     return KB_OK;
@@ -1011,7 +990,6 @@ static int registration_run(kb_registration *reg, const double *xyz, size_t n, k
     P.system_only = system_only ? 1 : 0;
     P.out_sys = reg->out.p + 16;
     P.out_ncorr = reg->iout.p + 1;
-    P.use_qcache = system_only ? 0 : 1;
     P.tag_base = ex.next_tag_base();
     P.team = ex.team;
     P.team.qrec = reg->ws.qrec.p;
@@ -1332,7 +1310,6 @@ static int pipeline_launch(kb_pipeline *p, long long id, const double *d_xyz, si
     P.max_iter = p->cfg.max_num_iterations;
     P.conv = p->cfg.convergence_criterion;
     P.min_motion_th = p->cfg.min_motion_th;
-    P.use_qcache = 1;
     P.tag_base = ex.next_tag_base();
     P.in_f32 = in_f32 ? 1 : 0;
     return ex.coop(k_register_frame, P, std::max<size_t>(QC_BYTES, ex.icp_smem), true);

@@ -153,7 +153,7 @@ __device__ unsigned g_kb_marks[256];
 __device__ __forceinline__ void kb_mark(unsigned code) {
     if (threadIdx.x == 0) *reinterpret_cast<volatile unsigned *>(&g_kb_marks[blockIdx.x & 255]) = code;
 }
-enum WatchdogCode { WD_GRID_BARRIER = 1, WD_ICP_GATHER16 = 2, WD_ICP_RESULT = 3, WD_TEAM_GATHER = 4, WD_NN_BULK = 5 };
+enum WatchdogCode { WD_GRID_BARRIER = 1, WD_ICP_GATHER16 = 2, WD_ICP_RESULT = 3, WD_TEAM_GATHER = 4 };
 
 __device__ __noinline__ bool kb_spin_giveup(unsigned spins, int code, unsigned a, unsigned b) {
     if (*reinterpret_cast<volatile unsigned *>(&g_kb_wd[0]) != 0u) return true;  // somebody gave up: everybody leaves
@@ -266,19 +266,25 @@ __device__ __forceinline__ int4 cas_slot(int4 *addr, int4 expected, int4 desired
     return o;
 }
 
-// lookup: slot index of voxel (x,y,z) or -1; *cnt = its point count
-__device__ __forceinline__ int map_find(const MapView &m, int x, int y, int z, int *cnt) {
-    unsigned h = mix_hash(x, y, z) & m.mask;
+// the collision chain of voxel (x,y,z) from bucket h, whose slot s is already loaded: slot index of the voxel or -1;
+// *cnt = its point count (untouched on a miss)
+__device__ __forceinline__ int map_find_from(const MapView &m, int x, int y, int z, unsigned h, int4 s, int *cnt) {
     for (unsigned probes = 0; probes <= m.mask; ++probes) {
-        const int4 s = m.slots[h];
         if (s.w == KB_EMPTY) return -1;
         if (s.w != KB_TOMB && s.x == x && s.y == y && s.z == z) {
             *cnt = s.w;
             return static_cast<int>(h);
         }
         h = (h + 1) & m.mask;
+        s = m.slots[h];
     }
     return -1;
+}
+
+// lookup: slot index of voxel (x,y,z) or -1; *cnt = its point count
+__device__ __forceinline__ int map_find(const MapView &m, int x, int y, int z, int *cnt) {
+    const unsigned h = mix_hash(x, y, z) & m.mask;
+    return map_find_from(m, x, y, z, h, m.slots[h], cnt);
 }
 
 // find-or-claim for AddPoints. New voxels are claimed with w = 0 by one 128-bit CAS; tombstones
@@ -839,14 +845,17 @@ __device__ __forceinline__ void nn_reduce(double &best, int &bseq, V3 &bp) {
     bseq = __shfl_sync(FULL, bseq, src);
 }
 
+// 2^-50: d2 > b2 * (1 + NN_TIE_REL) implies sqrt(d2) > sqrt(b2) after rounding. Within that bound two distinct
+// squares may round to the same root, and the reference's comparison of rounded roots has to be made.
+constexpr double NN_TIE_REL = 8.8817841970012523e-16;
+
 // candidate update with the reference's comparison (first strict minimum of the sqrt'ed norm),
-// computing the ~92-cycle DSQRT only when the squared distance could still win:
-// d2 > best_d2 * (1 + 2^-50) implies sqrt(d2) > sqrt(best_d2) after rounding.
+// computing the ~92-cycle DSQRT only when the squared distance could still win
 __device__ __forceinline__ void nn_consider(const V3 &c, const V3 &q, int seq, double &best, double &best_d2, int &bseq,
                                             V3 &bp) {
     const V3 df = c - q;
     const double d2 = sqnorm(df);
-    if (d2 <= best_d2 * (1.0 + 8.8817841970012523e-16)) {
+    if (d2 <= best_d2 * (1.0 + NN_TIE_REL)) {
         const double d = sqrt(d2);
         if (d < best) {
             best = d;
@@ -869,35 +878,49 @@ __device__ __forceinline__ NNResult nn_search_cached(const QCache &qc, const V3 
     return NNResult{best, bp, qc.full};
 }
 
-// Same result as nn_search_cached with ONE square root per query instead of one per lane and
-// candidate: the minimum is taken on squared distances (sqrt is monotone), which can only differ
-// from the reference's comparison of rounded sqrt values if some other candidate's squared
-// distance lies within a few ulps above the minimum (two distinct squares rounding to the same
-// root). That near-tie is detected — every lane also tracks its second smallest square — and
-// then the exact routine above is used instead (in practice: never).
-__device__ __forceinline__ NNResult nn_search_cached_fast(const QCache &qc, const V3 &q, int lane) {
-    double b2 = DBL_MAX, s2 = DBL_MAX;
-    int bseq = INT_MAX;
-    V3 bp{0, 0, 0};
-    const int total = qc.total;
-    for (int k = lane; k < total; k += 32) {
-        const V3 c{qc.pts[k][0], qc.pts[k][1], qc.pts[k][2]};
-        const double d2 = sqnorm(c - q);
+// ONE square root per query instead of one per lane and candidate: the minimum is taken on squared
+// distances (sqrt is monotone), which can only differ from the reference's comparison of rounded
+// sqrt values if some other candidate's squared distance lies within NN_TIE_REL above the minimum
+// (two distinct squares rounding to the same root). Every lane also tracks its second smallest
+// square, nn_reduce_near detects that near tie, and the caller then redoes the search with
+// nn_consider (in practice: never).
+struct NNMin {
+    double b2 = DBL_MAX;  // smallest square of this lane (after nn_reduce_near: of the warp)
+    double s2 = DBL_MAX;  // second smallest distinct square of this lane
+    int bseq = INT_MAX;   // sequence number (reference order) of the smallest
+    V3 bp{0, 0, 0};       // its point
+    __device__ __forceinline__ void add(double d2, int seq, const V3 &c) {
         if (d2 < b2) {
             s2 = b2;
             b2 = d2;
-            bseq = qc.seq[k];
+            bseq = seq;
             bp = c;
         } else if (d2 > b2 && d2 < s2) {
             s2 = d2;
         }
     }
-    const double mine = b2;
-    nn_reduce(b2, bseq, bp);  // b2 = warp minimum (exact ties: smallest reference sequence number)
-    const double lim = b2 * (1.0 + 8.8817841970012523e-16);
-    const bool near = (mine > b2 && mine <= lim) || (s2 <= lim);
-    if (__any_sync(FULL, near)) return nn_search_cached(qc, q, lane);
-    return NNResult{sqrt(b2), bp, qc.full};
+};
+
+// warp minimum of the lanes' accumulators (exact ties: smallest sequence number); true when another square of any
+// lane lies within NN_TIE_REL above it, i.e. the rounded roots have to be compared instead
+__device__ __forceinline__ bool nn_reduce_near(NNMin &a) {
+    const double mine = a.b2;
+    nn_reduce(a.b2, a.bseq, a.bp);
+    const double lim = a.b2 * (1.0 + NN_TIE_REL);
+    const bool near = (mine > a.b2 && mine <= lim) || (a.s2 <= lim);
+    return __any_sync(FULL, near);
+}
+
+// nn_search_cached with one square root per query
+__device__ __forceinline__ NNResult nn_search_cached_fast(const QCache &qc, const V3 &q, int lane) {
+    NNMin a;
+    const int total = qc.total;
+    for (int k = lane; k < total; k += 32) {
+        const V3 c{qc.pts[k][0], qc.pts[k][1], qc.pts[k][2]};
+        a.add(sqnorm(c - q), qc.seq[k], c);
+    }
+    if (nn_reduce_near(a)) return nn_search_cached(qc, q, lane);
+    return NNResult{sqrt(a.b2), a.bp, qc.full};
 }
 
 // 24-byte point record -> one 16-byte + one 8-byte load (records are 8-byte aligned, every other one 16-byte)
@@ -909,15 +932,44 @@ __device__ __forceinline__ V3 ld_point24(const double *rec) {
     return even ? V3{wide.x, wide.y, lone} : V3{lone, wide.x, wide.y};
 }
 
-// FLAT GATHER over the probed neighbourhood (per-lane cnt/slot of lanes 0..26): candidate j (reference order:
-// voxel_shifts order, then insertion order) goes to lane j % 32, so all loads of a round are independent — one
-// L2 round trip instead of one per occupied voxel. The minimum is taken on SQUARED distances (one sqrt per
-// query); if another candidate's square lies within a few ulps above the minimum (two squares that could round
-// to the same root) the search is redone comparing rounded roots exactly like the reference.
-// (the search proper: `w` already holds the slot / start / owner tables of the probed neighbourhood)
-__device__ __forceinline__ NNResult nn_flat_search_staged(const MapView &m, const V3 &q, int lane, WarpNN &w, int total);
+// lanes 0..26: point count and slot of neighbour voxel `lane` of voxel v (voxel_shifts order);
+// {0, -1} for an absent voxel and on lanes 27..31
+struct NNVoxel {
+    int cnt, slot;
+};
+__device__ __forceinline__ NNVoxel nn_probe27(const MapView &m, const int3 &v, int lane) {
+    NNVoxel r{0, -1};
+    if (lane < 27) r.slot = map_find(m, v.x + c_shifts[lane][0], v.y + c_shifts[lane][1], v.z + c_shifts[lane][2], &r.cnt);
+    return r;
+}
 
-__device__ __forceinline__ NNResult nn_flat_search(const MapView &m, const V3 &q, int lane, WarpNN &w, int cnt, int slot) {
+// general path (max_points_per_voxel > NN_FLAT_CAP): the warp walks the occupied voxels one after the other, lane i
+// taking point i of the block; sequence number = voxel * 1024 + point
+__device__ __forceinline__ NNResult nn_walk_voxels(const MapView &m, const V3 &q, int lane, int cnt, int slot) {
+    const int cap = m.cap;
+    double best = DBL_MAX, best_d2 = DBL_MAX;
+    int bseq = INT_MAX;
+    V3 bp{0, 0, 0};
+    unsigned occ = __ballot_sync(FULL, cnt > 0);
+    int total = 0;
+    while (occ) {
+        const int vi = __ffs(occ) - 1;
+        occ &= occ - 1;
+        const int c = __shfl_sync(FULL, cnt, vi);
+        const int s = __shfl_sync(FULL, slot, vi);
+        total += c;
+        const double *blk = m.points + static_cast<size_t>(s) * cap * 3;
+        for (int k = lane; k < c; k += 32)
+            nn_consider(V3{blk[3 * k], blk[3 * k + 1], blk[3 * k + 2]}, q, vi * 1024 + k, best, best_d2, bseq, bp);
+    }
+    nn_reduce(best, bseq, bp);
+    return NNResult{best, bp, total};
+}
+
+// flatten the probed neighbourhood (cnt / slot of lanes 0..26, cap <= NN_FLAT_CAP) into `w`: candidate j (reference
+// order: voxel_shifts order, then insertion order) is point j - w.start[v] of the block w.slot[v], v = w.owner[j].
+// Returns the number of candidates.
+__device__ __forceinline__ int nn_flatten(WarpNN &w, int lane, int cnt, int slot) {
     int incl = cnt;
 #pragma unroll
     for (int o = 1; o < 32; o <<= 1) {
@@ -933,14 +985,30 @@ __device__ __forceinline__ NNResult nn_flat_search(const MapView &m, const V3 &q
         for (int k = 0; k < cnt; ++k) w.owner[start + k] = static_cast<unsigned char>(lane);
     }
     __syncwarp();
-    return nn_flat_search_staged(m, q, lane, w, total);
+    return total;
 }
 
+// squared radius of the candidate lists: the candidates within d* + 2R of the query (QCache's exactness argument)
+__device__ __forceinline__ double nn_keep_thr2(double d, double cache_radius) {
+    const double thr = d + 2.0 * cache_radius;
+    return thr * thr * (1.0 + 1e-12);
+}
+
+// one step of an ordered warp compaction: the lanes with `keep` take positions count, count + 1, ... in lane order
+// (returned), and count grows by their number
+__device__ __forceinline__ int warp_compact(bool keep, int lane, int &count) {
+    const unsigned mask = __ballot_sync(FULL, keep);
+    const int pos = count + __popc(mask & ((1u << lane) - 1u));
+    count += __popc(mask);
+    return pos;
+}
+
+// FLAT GATHER over the flattened neighbourhood: candidate j goes to lane j % 32, so all loads of a round are
+// independent — one L2 round trip instead of one per occupied voxel. One sqrt per query (NNMin); on a near tie
+// the search is redone comparing rounded roots exactly like the reference.
 __device__ __forceinline__ NNResult nn_flat_search_staged(const MapView &m, const V3 &q, int lane, WarpNN &w, int total) {
     const int cap = m.cap;
-    double b2 = DBL_MAX, s2 = DBL_MAX;
-    int bseq = INT_MAX;
-    V3 bp{0, 0, 0};
+    NNMin a;
     constexpr int U = 2;
     for (int base = 0; base < total; base += 32 * U) {
         V3 c[U];
@@ -956,26 +1024,12 @@ __device__ __forceinline__ NNResult nn_flat_search_staged(const MapView &m, cons
         }
 #pragma unroll
         for (int u = 0; u < U; ++u)
-            if (ok[u]) {
-                const double d2 = sqnorm(c[u] - q);
-                if (d2 < b2) {
-                    s2 = b2;
-                    b2 = d2;
-                    bseq = base + u * 32 + lane;
-                    bp = c[u];
-                } else if (d2 > b2 && d2 < s2) {
-                    s2 = d2;
-                }
-            }
+            if (ok[u]) a.add(sqnorm(c[u] - q), base + u * 32 + lane, c[u]);
     }
-    const double mine = b2;
-    nn_reduce(b2, bseq, bp);
-    const double lim = b2 * (1.0 + 8.8817841970012523e-16);
-    const bool near = (mine > b2 && mine <= lim) || (s2 <= lim);
-    if (!__any_sync(FULL, near)) return NNResult{total > 0 ? sqrt(b2) : DBL_MAX, bp, total};
+    if (!nn_reduce_near(a)) return NNResult{total > 0 ? sqrt(a.b2) : DBL_MAX, a.bp, total};
     double best = DBL_MAX, best_d2 = DBL_MAX;
-    bseq = INT_MAX;
-    bp = V3{0, 0, 0};
+    int bseq = INT_MAX;
+    V3 bp{0, 0, 0};
     for (int j = lane; j < total; j += 32) {
         const int vi = w.owner[j];
         const double *pp = m.points + (static_cast<size_t>(w.slot[vi]) * cap + (j - w.start[vi])) * 3;
@@ -985,45 +1039,28 @@ __device__ __forceinline__ NNResult nn_flat_search_staged(const MapView &m, cons
     return NNResult{best, bp, total};
 }
 
+__device__ __forceinline__ NNResult nn_flat_search(const MapView &m, const V3 &q, int lane, WarpNN &w, int cnt, int slot) {
+    return nn_flat_search_staged(m, q, lane, w, nn_flatten(w, lane, cnt, slot));
+}
+
 __device__ __forceinline__ NNResult nn_search_warp(const MapView &m, const V3 &q, int lane, WarpNN &w,
                                                    QCache *fill = nullptr, double cache_radius = 0.0) {
     const int3 v = point_to_voxel(q.x, q.y, q.z, m.vdiv);
-    int cnt = 0, slot = -1;
-    if (lane < 27) {
-        slot = map_find(m, v.x + c_shifts[lane][0], v.y + c_shifts[lane][1], v.z + c_shifts[lane][2], &cnt);
-        if (slot < 0) cnt = 0;
-    }
+    const NNVoxel nv = nn_probe27(m, v, lane);
     const int cap = m.cap;
     if (cap > NN_FLAT_CAP) {
-        // general path (max_points_per_voxel > 32): walk the occupied voxels one after the other
-        double best = DBL_MAX, best_d2 = DBL_MAX;
-        int bseq = INT_MAX;
-        V3 bp{0, 0, 0};
-        unsigned occ = __ballot_sync(FULL, cnt > 0);
-        int total = 0;
-        while (occ) {
-            const int vi = __ffs(occ) - 1;
-            occ &= occ - 1;
-            const int c = __shfl_sync(FULL, cnt, vi);
-            const int s = __shfl_sync(FULL, slot, vi);
-            total += c;
-            const double *blk = m.points + static_cast<size_t>(s) * cap * 3;
-            for (int k = lane; k < c; k += 32)
-                nn_consider(V3{blk[3 * k], blk[3 * k + 1], blk[3 * k + 2]}, q, vi * 1024 + k, best, best_d2, bseq, bp);
-        }
+        const NNResult r = nn_walk_voxels(m, q, lane, nv.cnt, nv.slot);
         if (fill != nullptr && lane == 0) fill->total = -1;
-        nn_reduce(best, bseq, bp);
-        return NNResult{best, bp, total};
+        return r;
     }
-    const NNResult r = nn_flat_search(m, q, lane, w, cnt, slot);
+    const NNResult r = nn_flat_search(m, q, lane, w, nv.cnt, nv.slot);
     const double best = r.d;
     const int total = r.candidates;
     if (fill != nullptr) {
         // second pass (L1-hot): keep the candidates within d* + 2R of the query, in reference order
         int count = -1;
         if (best < DBL_MAX) {
-            const double thr = best + 2.0 * cache_radius;
-            const double thr2 = thr * thr * (1.0 + 1e-12);
+            const double thr2 = nn_keep_thr2(best, cache_radius);
             count = 0;
             constexpr int U2 = 4;
             for (int base = 0; base < total; base += 32 * U2) {
@@ -1037,15 +1074,13 @@ __device__ __forceinline__ NNResult nn_search_warp(const MapView &m, const V3 &q
                         c = ld_point24(m.points + (static_cast<size_t>(w.slot[vi]) * cap + (j - w.start[vi])) * 3);
                         keep = sqnorm(c - q) <= thr2;
                     }
-                    const unsigned mask = __ballot_sync(FULL, keep);
-                    const int pos = count + __popc(mask & ((1u << lane) - 1u));
+                    const int pos = warp_compact(keep, lane, count);
                     if (keep && pos < QC_MAX) {
                         fill->pts[pos][0] = c.x;
                         fill->pts[pos][1] = c.y;
                         fill->pts[pos][2] = c.z;
                         fill->seq[pos] = j;
                     }
-                    count += __popc(mask);
                 }
             }
             if (count > QC_MAX) count = -1;
@@ -1135,7 +1170,7 @@ __device__ __forceinline__ void icp_expand(const double a[NACC], double JTJ[36],
 // Reduction order is fixed: query-strided per warp -> 16-warp shuffle tree -> CTAs in order.
 __device__ __noinline__ void icp_queries(const Scratch &sc, Shared &sh, const MapView &m, const double *src, double *work, int n,
                             const SE3 &pending, double max_dist, double kscale, unsigned tag, bool dbg_on,
-                            QCache *qcache = nullptr, bool first = true, bool fill_first = false) {
+                            QCache *qcache, bool first) {
     // (copying sc / m / pending into locals was measured: -0.6 us on the query phase but slower overall, the
     // extra live registers spill in the search code)
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -1174,10 +1209,9 @@ __device__ __noinline__ void icp_queries(const Scratch &sc, Shared &sh, const Ma
                 (qc->any_voxel || (qc->vx == v.x && qc->vy == v.y && qc->vz == v.z)))
                 r = nn_search_cached_fast(*qc, p, lane), ++n_hit;
             else {
-                // whether filling already pays off on the first iteration depends on the size of the first step:
-                // with a good constant-velocity prediction (steady driving) most caches survive it (measured
-                // -4 us/scan), after a poor one they are refilled on iteration 1 anyway (fill_first = false)
-                r = nn_search_warp(m, p, lane, sh.wnn[warp], (first && !fill_first) ? nullptr : qc, radius);
+                // (filled on the first iteration too: with a good constant-velocity prediction (steady driving) most
+                // caches survive the first step, measured -4 us/scan)
+                r = nn_search_warp(m, p, lane, sh.wnn[warp], qc, radius);
                 ++n_fill;
                 n_over += (qc->total < 0 && r.d < DBL_MAX) ? 1 : 0;
             }
@@ -1276,7 +1310,7 @@ __device__ __forceinline__ void icp_gather(const Scratch &sc, Shared &sh, unsign
 // ------------------------------------------------------------------------------------------
 __device__ __noinline__ void op_icp(Grid &g, const Scratch &sc, Shared &sh, const MapView &m, const double *src, double *work,
                        int n, const SE3 &guess, double max_dist, double kscale, int max_iter, double conv,
-                       QCache *qcache, unsigned tag_base, bool fill_first = true) {
+                       QCache *qcache, unsigned tag_base) {
     (void)g;
     if (__ldcg(&m.counters[C_LIVE]) == 0 || max_iter <= 0) {  // voxel_map.Empty() -> initial_guess (:143)
         __syncthreads();
@@ -1302,7 +1336,7 @@ __device__ __noinline__ void op_icp(Grid &g, const Scratch &sc, Shared &sh, cons
         if (sc.profile && blockIdx.x == 0 && threadIdx.x == 0 && j < 20) sc.dbg[41 + j] = globaltimer_ns();
         const bool dbg_on = sc.profile && (j == 4);
         const unsigned tag = tag_base + static_cast<unsigned>(j) + 1u;
-        icp_queries(sc, sh, m, j == 0 ? src : work, work, n, pending, max_dist, kscale, tag, dbg_on, qcache, j == 0, fill_first);
+        icp_queries(sc, sh, m, j == 0 ? src : work, work, n, pending, max_dist, kscale, tag, dbg_on, qcache, j == 0);
         if (dbg_on) { KB_CYC(sc, 4); }
         icp_gather(sc, sh, tag, gs);  // group leaders and the coordinator work, everybody else falls through
         if (blockIdx.x == 0) {

@@ -35,7 +35,7 @@ static_assert(TQ_MAX * TRED_STRIDE * 8 <= DS_MAX_CHUNKS * 4, "the reduction scra
 // reference's visiting order (voxel_shifts order, then insertion order), so the first strict minimum over the
 // list is the reference's answer, ties included.
 struct QList {
-    int count;      // >= 0: idx[0..count) valid; -1: not cacheable (too many candidates / max_points_per_voxel > 32)
+    int count;      // >= 0: idx[0..count) valid; -1: not cacheable (too many candidates)
     int full;       // points of the whole 27-voxel neighbourhood (bookkeeping of algorithmic bytes)
     int vx, vy, vz; // voxel at fill time
     int pad[3];
@@ -123,159 +123,94 @@ __device__ __forceinline__ int icp_team_size(int n, int q_per_cta, int grid, int
 // ONE pass over the neighbourhood: every lane keeps the squared distances and point indices of its <= 8 candidates
 // in registers (all loads of the neighbourhood are in flight together: one L2 round trip), the warp takes the
 // minimum, and the list is filtered from the registers. Neighbourhoods with more than 256 points take two passes.
+// Only for maps with max_points_per_voxel <= NN_FLAT_CAP: the team does not run on others.
 constexpr int NNL_R = 8;
 __device__ __noinline__ NNResult nn_search_list(const MapView &m, const V3 &q, int lane, WarpNN &w, QList *out,
                                                 double cache_radius) {
     const int3 v = point_to_voxel(q.x, q.y, q.z, m.vdiv);
-    int cnt = 0, slot = -1;
-    if (lane < 27) {
-        slot = map_find(m, v.x + c_shifts[lane][0], v.y + c_shifts[lane][1], v.z + c_shifts[lane][2], &cnt);
-        if (slot < 0) cnt = 0;
-    }
+    const NNVoxel nv = nn_probe27(m, v, lane);
     const int cap = m.cap;
+    // candidate j (reference order) -> lane j % 32, register j / 32
+    const int total = nn_flatten(w, lane, nv.cnt, nv.slot);
     NNResult r;
-    int count = -1;
-    if (cap > NN_FLAT_CAP) {
-        // general path (max_points_per_voxel > 32): no list, the point is searched again every iteration
-        double best = DBL_MAX, best_d2 = DBL_MAX;
-        int bseq = INT_MAX;
-        V3 bp{0, 0, 0};
-        unsigned occ = __ballot_sync(FULL, cnt > 0);
-        int total = 0;
-        while (occ) {
-            const int vi = __ffs(occ) - 1;
-            occ &= occ - 1;
-            const int c = __shfl_sync(FULL, cnt, vi);
-            const int s = __shfl_sync(FULL, slot, vi);
-            total += c;
-            const double *blk = m.points + static_cast<size_t>(s) * cap * 3;
-            for (int k = lane; k < c; k += 32)
-                nn_consider(V3{blk[3 * k], blk[3 * k + 1], blk[3 * k + 2]}, q, vi * 1024 + k, best, best_d2, bseq, bp);
-        }
-        nn_reduce(best, bseq, bp);
-        r = NNResult{best, bp, total};
-    } else {
-        // flatten the neighbourhood over the lanes: candidate j (reference order) -> lane j % 32, register j / 32
-        int incl = cnt;
+    int count = 0;  // (an empty neighbourhood stays empty while the point stays in its voxel)
+    if (total <= 32 * NNL_R) {
+        double d2[NNL_R];
+        int gi[NNL_R];
 #pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            const int t = __shfl_up_sync(FULL, incl, o);
-            if (lane >= o) incl += t;
-        }
-        const int start = incl - cnt;
-        const int total = __shfl_sync(FULL, incl, 31);
-        __syncwarp();
-        if (lane < 27) {
-            w.slot[lane] = slot;
-            w.start[lane] = start;
-            for (int k = 0; k < cnt; ++k) w.owner[start + k] = static_cast<unsigned char>(lane);
-        }
-        __syncwarp();
-        if (total <= 32 * NNL_R) {
-            double d2[NNL_R];
-            int gi[NNL_R];
+        for (int h = 0; h < NNL_R; h += 4) {  // (the loads of both halves are independent: one round trip)
+            V3 c[4];
 #pragma unroll
-            for (int h = 0; h < NNL_R; h += 4) {  // (the loads of both halves are independent: one round trip)
-                V3 c[4];
-#pragma unroll
-                for (int u = 0; u < 4; ++u) {
-                    const int j = (h + u) * 32 + lane;
-                    gi[h + u] = -1;
-                    if (j < total) {
-                        const int vi = w.owner[j];
-                        gi[h + u] = w.slot[vi] * cap + (j - w.start[vi]);
-                        c[u] = ld_point24(m.points + static_cast<size_t>(gi[h + u]) * 3);
-                    }
+            for (int u = 0; u < 4; ++u) {
+                const int j = (h + u) * 32 + lane;
+                gi[h + u] = -1;
+                if (j < total) {
+                    const int vi = w.owner[j];
+                    gi[h + u] = w.slot[vi] * cap + (j - w.start[vi]);
+                    c[u] = ld_point24(m.points + static_cast<size_t>(gi[h + u]) * 3);
                 }
-#pragma unroll
-                for (int u = 0; u < 4; ++u) d2[h + u] = (gi[h + u] >= 0) ? sqnorm(c[u] - q) : DBL_MAX;
             }
-            double b2 = DBL_MAX, s2 = DBL_MAX;
-            int bseq = INT_MAX, bg = -1;
+#pragma unroll
+            for (int u = 0; u < 4; ++u) d2[h + u] = (gi[h + u] >= 0) ? sqnorm(c[u] - q) : DBL_MAX;
+        }
+        NNMin a;  // (no points: the winner's is re-read below, it is L1-hot)
+#pragma unroll
+        for (int u = 0; u < NNL_R; ++u) a.add(d2[u], u * 32 + lane, V3{0, 0, 0});
+        if (!nn_reduce_near(a)) {
+            V3 bp{0, 0, 0};
+            if (total > 0) {
+                const int vi = w.owner[a.bseq];
+                bp = ld_point24(m.points + static_cast<size_t>(w.slot[vi] * cap + (a.bseq - w.start[vi])) * 3);
+            }
+            r = NNResult{total > 0 ? sqrt(a.b2) : DBL_MAX, bp, total};
+        } else {  // near tie of squared distances: compare rounded roots in reference order, like the reference
+            double best = DBL_MAX, best_d2 = DBL_MAX;
+            int bseq = INT_MAX;
+            V3 bp{0, 0, 0};
+#pragma unroll
+            for (int u = 0; u < NNL_R; ++u)
+                if (gi[u] >= 0) {
+                    const double *pp = m.points + static_cast<size_t>(gi[u]) * 3;
+                    nn_consider(V3{pp[0], pp[1], pp[2]}, q, u * 32 + lane, best, best_d2, bseq, bp);
+                }
+            nn_reduce(best, bseq, bp);
+            r = NNResult{best, bp, total};
+        }
+        // the candidates within d* + 2R of the point, in reference order
+        if (r.d < DBL_MAX) {
+            const double thr2 = nn_keep_thr2(r.d, cache_radius);
 #pragma unroll
             for (int u = 0; u < NNL_R; ++u) {
-                if (d2[u] < b2) {
-                    s2 = b2;
-                    b2 = d2[u];
-                    bseq = u * 32 + lane;
-                    bg = gi[u];
-                } else if (d2[u] > b2 && d2[u] < s2) {
-                    s2 = d2[u];
+                if (u * 32 < total) {  // warp-uniform
+                    const bool keep = d2[u] <= thr2;  // (DBL_MAX where there is no candidate)
+                    const int pos = warp_compact(keep, lane, count);
+                    if (keep && pos < QC_MAX) out->idx[pos] = gi[u];
                 }
             }
-            const double mine = b2;
-            V3 bp{0, 0, 0};
-            nn_reduce(b2, bseq, bp);  // (bp is a dummy: the winner's point is re-read below, it is L1-hot)
-            const double lim = b2 * (1.0 + 8.8817841970012523e-16);
-            const bool near = (mine > b2 && mine <= lim) || (s2 <= lim);
-            if (!__any_sync(FULL, near)) {
-                if (total > 0) {
-                    const int gw = __shfl_sync(FULL, bg, bseq & 31);  // the winning lane's own minimum IS the warp minimum
-                    bp = ld_point24(m.points + static_cast<size_t>(gw) * 3);
-                }
-                r = NNResult{total > 0 ? sqrt(b2) : DBL_MAX, bp, total};
-            } else {  // near tie of squared distances: compare rounded roots in reference order, like the reference
-                double best = DBL_MAX, best_d2 = DBL_MAX;
-                bseq = INT_MAX;
-                bp = V3{0, 0, 0};
+        }
+    } else {
+        r = nn_flat_search_staged(m, q, lane, w, total);
+        if (r.d < DBL_MAX) {  // second pass (L1-hot)
+            const double thr2 = nn_keep_thr2(r.d, cache_radius);
+            constexpr int U2 = 4;
+            for (int base = 0; base < total; base += 32 * U2) {
 #pragma unroll
-                for (int u = 0; u < NNL_R; ++u)
-                    if (gi[u] >= 0) {
-                        const double *pp = m.points + static_cast<size_t>(gi[u]) * 3;
-                        nn_consider(V3{pp[0], pp[1], pp[2]}, q, u * 32 + lane, best, best_d2, bseq, bp);
+                for (int u = 0; u < U2; ++u) {
+                    const int j = base + u * 32 + lane;
+                    bool keep = false;
+                    int g = 0;
+                    if (j < total) {
+                        const int vi = w.owner[j];
+                        g = w.slot[vi] * cap + (j - w.start[vi]);
+                        keep = sqnorm(ld_point24(m.points + static_cast<size_t>(g) * 3) - q) <= thr2;
                     }
-                nn_reduce(best, bseq, bp);
-                r = NNResult{best, bp, total};
-            }
-            // the candidates within d* + 2R of the point, in reference order
-            if (r.d < DBL_MAX) {
-                const double thr = r.d + 2.0 * cache_radius;
-                const double thr2 = thr * thr * (1.0 + 1e-12);
-                count = 0;
-#pragma unroll
-                for (int u = 0; u < NNL_R; ++u) {
-                    if (u * 32 < total) {  // warp-uniform
-                        const bool keep = d2[u] <= thr2;  // (DBL_MAX where there is no candidate)
-                        const unsigned mask = __ballot_sync(FULL, keep);
-                        const int pos = count + __popc(mask & ((1u << lane) - 1u));
-                        if (keep && pos < QC_MAX) out->idx[pos] = gi[u];
-                        count += __popc(mask);
-                    }
+                    const int pos = warp_compact(keep, lane, count);
+                    if (keep && pos < QC_MAX) out->idx[pos] = g;
                 }
-                if (count > QC_MAX) count = -1;
-            } else {
-                count = 0;  // empty neighbourhood: stays empty while the point stays in its voxel
-            }
-        } else {
-            r = nn_flat_search_staged(m, q, lane, w, total);
-            if (r.d < DBL_MAX) {  // second pass (L1-hot)
-                const double thr = r.d + 2.0 * cache_radius;
-                const double thr2 = thr * thr * (1.0 + 1e-12);
-                count = 0;
-                constexpr int U2 = 4;
-                for (int base = 0; base < total; base += 32 * U2) {
-#pragma unroll
-                    for (int u = 0; u < U2; ++u) {
-                        const int j = base + u * 32 + lane;
-                        bool keep = false;
-                        int g = 0;
-                        if (j < total) {
-                            const int vi = w.owner[j];
-                            g = w.slot[vi] * cap + (j - w.start[vi]);
-                            keep = sqnorm(ld_point24(m.points + static_cast<size_t>(g) * 3) - q) <= thr2;
-                        }
-                        const unsigned mask = __ballot_sync(FULL, keep);
-                        const int pos = count + __popc(mask & ((1u << lane) - 1u));
-                        if (keep && pos < QC_MAX) out->idx[pos] = g;
-                        count += __popc(mask);
-                    }
-                }
-                if (count > QC_MAX) count = -1;
-            } else {
-                count = 0;
             }
         }
     }
+    if (count > QC_MAX) count = -1;
     if (lane == 0) {
         out->count = count;
         out->full = r.candidates;
@@ -560,7 +495,7 @@ __device__ __forceinline__ void team_queries(uint4 *ll, Shared &sh, const MapVie
         KB_WCYC(2);
         // two squares within a few ulps could round to the same root: then compare rounded roots in reference
         // order like GetClosestNeighbor does (in practice never)
-        const bool near = cnt > 0 && s2 <= b2 * (1.0 + 8.8817841970012523e-16);
+        const bool near = cnt > 0 && s2 <= b2 * (1.0 + NN_TIE_REL);
         if (__any_sync(FULL, near)) {
             tq_exact_nn(sm, li, l4, cnt, near, p.x, p.y, p.z);
             if (near) {

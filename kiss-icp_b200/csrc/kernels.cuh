@@ -77,7 +77,6 @@ struct FrameParams {
     double max_range, min_range, voxel_size;
     int max_iter;
     double conv, min_motion_th;
-    int use_qcache;
     int icp_team_q;  // source points per CTA of the ICP team; 0: whole-grid loop (op_icp)
     unsigned tag_base;
 };
@@ -211,7 +210,7 @@ __global__ void __launch_bounds__(BLOCK, 1) k_register_frame(const FrameParams P
         __syncthreads();
     } else {
         op_icp(g, P.sc, sh, P.m, fr.src, P.ws.work, n_src, guess, 3.0 * sigma, sigma, P.max_iter, P.conv,
-               P.use_qcache ? reinterpret_cast<QCache *>(kb_dyn_smem) : nullptr, P.tag_base);
+               reinterpret_cast<QCache *>(kb_dyn_smem), P.tag_base);
     }
     const SE3 new_pose = sh.result;
     const int iters = sh.iters;
@@ -342,7 +341,6 @@ struct IcpParams {
     int system_only;
     double *out_sys;
     int *out_ncorr;
-    int use_qcache;
     unsigned tag_base;
     TeamScratch team;
     int icp_team_q;  // source points per CTA of the ICP team; 0: whole-grid loop
@@ -352,7 +350,8 @@ __global__ void __launch_bounds__(BLOCK, 1) k_icp(const IcpParams P) {
     Grid g;
     g.init(P.sc.bar);
     if (P.system_only) {
-        icp_queries(P.sc, sh, P.m, P.src, P.work, P.n, se3_identity(), P.max_dist, P.kscale, P.tag_base + 1u, false);
+        icp_queries(P.sc, sh, P.m, P.src, P.work, P.n, se3_identity(), P.max_dist, P.kscale, P.tag_base + 1u, false,
+                    nullptr, true);
         icp_gather(P.sc, sh, P.tag_base + 1u, icp_group_size());
         if (blockIdx.x == 0) {
             if (threadIdx.x == 0) {
@@ -363,7 +362,7 @@ __global__ void __launch_bounds__(BLOCK, 1) k_icp(const IcpParams P) {
         return;
     }
     int T = 0;
-    if (__ldcg(&P.m.counters[C_LIVE]) != 0 && P.max_iter > 0 && P.icp_team_q > 0 && P.use_qcache && P.m.cap <= NN_FLAT_CAP &&
+    if (__ldcg(&P.m.counters[C_LIVE]) != 0 && P.max_iter > 0 && P.icp_team_q > 0 && P.m.cap <= NN_FLAT_CAP &&
         (static_cast<unsigned long long>(P.m.mask) + 1) * P.m.cap < (1ull << 31)) {
         T = icp_team_size(P.n, P.icp_team_q, static_cast<int>(gridDim.x), P.team.smem_bytes);
     }
@@ -375,7 +374,7 @@ __global__ void __launch_bounds__(BLOCK, 1) k_icp(const IcpParams P) {
                     kb_dyn_smem, T, P.tag_base);
     } else {
         op_icp(g, P.sc, sh, P.m, P.src, P.work, P.n, P.guess, P.max_dist, P.kscale, P.max_iter, P.conv,
-               P.use_qcache ? reinterpret_cast<QCache *>(kb_dyn_smem) : nullptr, P.tag_base);
+               reinterpret_cast<QCache *>(kb_dyn_smem), P.tag_base);
     }
     if (blockIdx.x == 0 && threadIdx.x == 0) {
         se3_to_matrix(sh.result, P.out_pose);
@@ -472,43 +471,11 @@ __device__ __forceinline__ void nn_issue(const MapView &m, const double *__restr
 // finish the probe started by nn_issue (collision chain), then gather + reduce exactly like nn_search_warp
 __device__ __forceinline__ NNResult nn_finish(const MapView &m, const NNProbe &pr, int lane, WarpNN &w) {
     int cnt = 0, slot = -1;
-    if (lane < 27) {
-        const int x = pr.v.x + c_shifts[lane][0], y = pr.v.y + c_shifts[lane][1], z = pr.v.z + c_shifts[lane][2];
-        unsigned h = pr.h;
-        int4 s = pr.s;
-        for (unsigned probes = 0; probes <= m.mask; ++probes) {
-            if (s.w == KB_EMPTY) break;
-            if (s.w != KB_TOMB && s.x == x && s.y == y && s.z == z) {
-                cnt = s.w;
-                slot = static_cast<int>(h);
-                break;
-            }
-            h = (h + 1) & m.mask;
-            s = m.slots[h];
-        }
-    }
-    const V3 q = pr.q;
-    const int cap = m.cap;
-    if (cap <= NN_FLAT_CAP) return nn_flat_search(m, q, lane, w, cnt, slot);
-    double best = DBL_MAX, best_d2 = DBL_MAX;
-    int bseq = INT_MAX;
-    V3 bp{0, 0, 0};
-    int total = 0;
-    {
-        unsigned occ = __ballot_sync(FULL, cnt > 0);
-        while (occ) {
-            const int vi = __ffs(occ) - 1;
-            occ &= occ - 1;
-            const int c = __shfl_sync(FULL, cnt, vi);
-            const int sidx = __shfl_sync(FULL, slot, vi);
-            total += c;
-            const double *blk = m.points + static_cast<size_t>(sidx) * cap * 3;
-            for (int k = lane; k < c; k += 32)
-                nn_consider(V3{blk[3 * k], blk[3 * k + 1], blk[3 * k + 2]}, q, vi * 1024 + k, best, best_d2, bseq, bp);
-        }
-    }
-    nn_reduce(best, bseq, bp);
-    return NNResult{best, bp, total};
+    if (lane < 27)
+        slot = map_find_from(m, pr.v.x + c_shifts[lane][0], pr.v.y + c_shifts[lane][1], pr.v.z + c_shifts[lane][2], pr.h,
+                             pr.s, &cnt);
+    if (m.cap <= NN_FLAT_CAP) return nn_flat_search(m, pr.q, lane, w, cnt, slot);
+    return nn_walk_voxels(m, pr.q, lane, cnt, slot);
 }
 
 template <bool COUNT>
@@ -537,217 +504,6 @@ __global__ void __launch_bounds__(256, 4) k_nn_query(const MapView m, const doub
     }
     if (COUNT && lane == 0 && cand) atomicAdd(cand_total, cand);
 }
-
-// ---- batched GetClosestNeighbor with the candidate blocks STAGED BY BULK ASYNC COPIES (default for config 5) --------
-// k_nn_query is bound by bytes in flight (profiles/README.md): a warp can only have outstanding what fits in its
-// registers (64 candidates = 1.5 KB) and the loads sit on its dependent path. Here every occupied neighbour voxel's
-// point block goes to the warp's 8 KB shared-memory buffer with ONE cp.async.bulk (UBLKCP; blocks are 16-byte
-// aligned: slot * cap * 24 with cap even), completion is counted by the warp's mbarrier, and while the ~3.5 KB of a
-// query are in flight the warp walks the NEXT query's probe chain; the reduction then reads dense 24-byte slots from
-// shared memory (conflict-free: 16 lanes x 24 B cover 16 distinct 8-byte bank pairs). 24 warps per SM x 3.5 KB in
-// flight is what Little's law asks for at the measured HBM bandwidth. (A variant with two buffers per warp — query
-// i + 1 copied while query i is reduced, 16 warps per SM — was measured slower: 1.77 ms vs 1.59 ms.) Voxels with an odd count are copied with one
-// extra point (48-byte multiples); that pad slot is overwritten with +inf coordinates before the reduction, so it can
-// never win. Slot numbers increase with the reference's visiting order, so ties resolve like in k_nn_query.
-constexpr int NNB_BUF = 8192;             // bytes per warp: 341 candidate slots (p99 of a KITTI-scale neighbourhood ~300)
-constexpr int NNB_SLOTS = NNB_BUF / 24;
-constexpr int NNB_WARPS = 8;              // 256 threads, 3 CTAs per SM
-
-__device__ __forceinline__ unsigned smem_u32(const void *p) { return static_cast<unsigned>(__cvta_generic_to_shared(p)); }
-__device__ __forceinline__ void mbar_init(unsigned bar, unsigned count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(unsigned bar, unsigned bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void bulk_g2s(unsigned dst, const void *src, unsigned bytes, unsigned bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst),
-                 "l"(src), "r"(bytes), "r"(bar)
-                 : "memory");
-}
-__device__ __forceinline__ bool mbar_try_wait(unsigned bar, unsigned parity) {
-    unsigned ok;
-    asm volatile(
-        "{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(ok)
-        : "r"(bar), "r"(parity)
-        : "memory");
-    return ok != 0;
-}
-
-// what a warp remembers about the query whose blocks are in flight
-struct NNStaged {
-    V3 q;
-    int cnt, slot;     // this lane's neighbour voxel (lanes 0..26)
-    int startp;        // its first candidate slot in the buffer (even)
-    int totalp, real;  // padded / real candidates of the neighbourhood
-    bool staged;       // blocks were copied to shared memory (else: the register path handles it)
-};
-
-// walk the collision chain of the probe started by nn_issue -> this lane's (cnt, slot)
-__device__ __forceinline__ void nn_probe_finish(const MapView &m, const NNProbe &pr, int lane, int *cnt_out, int *slot_out) {
-    int cnt = 0, slot = -1;
-    if (lane < 27) {
-        const int x = pr.v.x + c_shifts[lane][0], y = pr.v.y + c_shifts[lane][1], z = pr.v.z + c_shifts[lane][2];
-        unsigned h = pr.h;
-        int4 s = pr.s;
-        for (unsigned probes = 0; probes <= m.mask; ++probes) {
-            if (s.w == KB_EMPTY) break;
-            if (s.w != KB_TOMB && s.x == x && s.y == y && s.z == z) {
-                cnt = s.w;
-                slot = static_cast<int>(h);
-                break;
-            }
-            h = (h + 1) & m.mask;
-            s = m.slots[h];
-        }
-    }
-    *cnt_out = cnt;
-    *slot_out = slot;
-}
-
-template <bool COUNT>
-__global__ void __launch_bounds__(NNB_WARPS * 32, 3) k_nn_query_bulk(const MapView m, const double *__restrict__ q, size_t n,
-                                                                    double *__restrict__ out_p, double *__restrict__ out_d,
-                                                                    unsigned long long *cand_total) {
-    extern __shared__ __align__(128) unsigned char nnb_smem[];  // NNB_WARPS x NNB_BUF
-    __shared__ __align__(8) unsigned long long bars[NNB_WARPS];
-    __shared__ WarpNN wnn[NNB_WARPS];  // neighbourhoods that do not fit the buffer take k_nn_query's register path
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    unsigned char *buf = nnb_smem + warp * NNB_BUF;
-    const unsigned bar = smem_u32(&bars[warp]);
-    if (lane == 0) mbar_init(bar, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    __syncwarp();
-    unsigned phase = 0;
-    const size_t gw = (blockIdx.x * static_cast<size_t>(blockDim.x) + threadIdx.x) >> 5;
-    const size_t nw = (static_cast<size_t>(gridDim.x) * blockDim.x) >> 5;
-    const int cap = m.cap;
-    const double inf = __longlong_as_double(0x7ff0000000000000LL);
-    unsigned long long cand = 0;
-
-    // offsets of the neighbourhood in the buffer + the copies themselves
-    auto stage = [&](const V3 &qq, int cnt, int slot) -> NNStaged {
-        NNStaged st;
-        st.q = qq;
-        st.cnt = cnt;
-        st.slot = slot;
-        const int pc = (cnt + 1) & ~1;
-        int incl = pc, real = cnt;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            const int t = __shfl_up_sync(FULL, incl, o);
-            if (lane >= o) incl += t;
-            real += __shfl_xor_sync(FULL, real, o);
-        }
-        st.startp = incl - pc;
-        st.totalp = __shfl_sync(FULL, incl, 31);
-        st.real = real;
-        st.staged = st.totalp > 0 && st.totalp <= NNB_SLOTS;
-        if (st.staged) {
-            // the previous query's shared-memory reads and pad writes (generic proxy) come before these async-proxy writes
-            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-            if (lane == 0) mbar_expect_tx(bar, static_cast<unsigned>(st.totalp) * 24u);
-            __syncwarp();
-            if (cnt > 0)
-                bulk_g2s(smem_u32(buf + st.startp * 24), m.points + static_cast<size_t>(slot) * cap * 3,
-                         static_cast<unsigned>(pc) * 24u, bar);
-        }
-        return st;
-    };
-
-    NNProbe nxt;
-    NNStaged cur;
-    if (gw < n) {
-        NNProbe first;
-        nn_issue(m, q, gw, lane, first);
-        int c0, s0;
-        nn_probe_finish(m, first, lane, &c0, &s0);
-        cur = stage(first.q, c0, s0);
-        if (gw + nw < n) nn_issue(m, q, gw + nw, lane, nxt);
-    }
-    for (size_t i = gw; i < n; i += nw) {
-        const bool more = i + nw < n;
-        // (1) while the blocks of query i fly: the probe chain of query i + 1, first probes of query i + 2
-        int c1 = 0, s1 = -1;
-        V3 q1{0.0, 0.0, 0.0};
-        if (more) {
-            nn_probe_finish(m, nxt, lane, &c1, &s1);
-            q1 = nxt.q;
-            if (i + 2 * nw < n) nn_issue(m, q, i + 2 * nw, lane, nxt);
-        }
-        // (2) reduce query i
-        NNResult r;
-        if (cur.staged) {
-            unsigned spins = 0;
-            while (!mbar_try_wait(bar, phase)) {
-                if (kb_spin_check(spins, WD_NN_BULK, static_cast<unsigned>(i), phase)) break;
-            }
-            phase ^= 1u;
-            if (cur.cnt & 1) {  // pad slot of an odd voxel: can never win
-                double *pad = reinterpret_cast<double *>(buf + (cur.startp + cur.cnt) * 24);
-                pad[0] = inf;
-                pad[1] = inf;
-                pad[2] = inf;
-            }
-            __syncwarp();
-            const V3 qq = cur.q;
-            double b2 = DBL_MAX, s2 = DBL_MAX;
-            int bseq = INT_MAX;
-            V3 bp{0.0, 0.0, 0.0};
-            for (int sidx = lane; sidx < cur.totalp; sidx += 32) {
-                const double *pp = reinterpret_cast<const double *>(buf + sidx * 24);
-                const V3 c{pp[0], pp[1], pp[2]};
-                const double d2 = sqnorm(c - qq);
-                if (d2 < b2) {
-                    s2 = b2;
-                    b2 = d2;
-                    bseq = sidx;
-                    bp = c;
-                } else if (d2 > b2 && d2 < s2) {
-                    s2 = d2;
-                }
-            }
-            const double mine = b2;
-            nn_reduce(b2, bseq, bp);
-            const double lim = b2 * (1.0 + 8.8817841970012523e-16);
-            const bool near = (mine > b2 && mine <= lim) || (s2 <= lim);
-            if (!__any_sync(FULL, near)) {
-                r = NNResult{sqrt(b2), bp, cur.real};
-            } else {  // near tie of squared distances: compare rounded roots in reference order, like nn_flat_search
-                double best = DBL_MAX, best_d2 = DBL_MAX;
-                bseq = INT_MAX;
-                bp = V3{0.0, 0.0, 0.0};
-                for (int sidx = lane; sidx < cur.totalp; sidx += 32) {
-                    const double *pp = reinterpret_cast<const double *>(buf + sidx * 24);
-                    nn_consider(V3{pp[0], pp[1], pp[2]}, qq, sidx, best, best_d2, bseq, bp);
-                }
-                nn_reduce(best, bseq, bp);
-                r = NNResult{best, bp, cur.real};
-            }
-            __syncwarp();  // every lane is done with the buffer before the next query's copies land in it
-        } else if (cur.totalp == 0) {
-            r = NNResult{DBL_MAX, V3{0.0, 0.0, 0.0}, 0};
-        } else {
-            r = nn_flat_search(m, cur.q, lane, wnn[warp], cur.cnt, cur.slot);
-        }
-        if (lane == 0) {
-            out_p[3 * i] = r.p.x;
-            out_p[3 * i + 1] = r.p.y;
-            out_p[3 * i + 2] = r.p.z;
-            out_d[i] = r.d;
-        }
-        if (COUNT) cand += r.candidates;
-        // (3) copies of query i + 1
-        if (more) cur = stage(q1, c1, s1);
-    }
-    if (COUNT && lane == 0 && cand) atomicAdd(cand_total, cand);
-}
-
-// (Measured and removed in round 2: the same pipeline with per-lane 16-byte cp.async (LDGSTS) instead of the bulk copies, a
-// branch-free two-candidates-per-trip walk and the winning lane writing the answer itself: ~470 instead of ~800 warp
-// instructions per query, bit-identical answers, and SLOWER - 2.02 ms against 1.70 ms (bulk) and 1.59 ms (registers) on
-// the same box. Instruction count is not what limits this kernel.)
 
 // export of live voxels (checkpoint / Pointcloud / tests): ordered two-pass compaction by slot
 struct ExportParams {

@@ -150,14 +150,15 @@ def test_map_growth_and_tombstone_rehash(K, O):
 
 
 def test_closest_neighbors_bit_exact(K, O, lidar):
-    g, o = build_pair(K, O, lidar, 5)
-    p3, _ = lidar.scan(3)
-    q = O.se3_act(np.linalg.inv(lidar.pose(0)) @ lidar.pose(3), p3) + rng.normal(size=p3.shape) * 0.2
-    q = np.concatenate([q, [[1e4, 1e4, 1e4]]])
-    ap, ad = g.closest_neighbors(q)
-    bp, bd = o.closest_neighbors(q)
-    assert np.array_equal(ap, bp) and np.array_equal(ad, bd)
-    assert ad[-1] == DBL_MAX and np.array_equal(ap[-1], [0, 0, 0])  # VoxelHashMap.cpp:51-52
+    for cap in (20, 32, 33, 37, 64):  # max_points_per_voxel <= 32: flat gather, > 32: voxel-by-voxel walk
+        g, o = build_pair(K, O, lidar, 5, cap=cap)
+        p3, _ = lidar.scan(3)
+        q = O.se3_act(np.linalg.inv(lidar.pose(0)) @ lidar.pose(3), p3) + rng.normal(size=p3.shape) * 0.2
+        q = np.concatenate([q, [[1e4, 1e4, 1e4]]])
+        ap, ad = g.closest_neighbors(q)
+        bp, bd = o.closest_neighbors(q)
+        assert np.array_equal(ap, bp) and np.array_equal(ad, bd), cap
+        assert ad[-1] == DBL_MAX and np.array_equal(ap[-1], [0, 0, 0]), cap  # VoxelHashMap.cpp:51-52
 
 
 def test_closest_neighbors_golden_and_ties(K, golden):
@@ -171,6 +172,14 @@ def test_closest_neighbors_golden_and_ties(K, golden):
     t.add_points(np.array([[1.25, 0.5, 0.5], [-0.25, 0.5, 0.5], [0.5, 1.25, 0.5]]))
     p, d = t.closest_neighbors(np.array([[0.5, 0.5, 0.5]]))
     assert d[0] == 0.75 and np.array_equal(p[0], [1.25, 0.5, 0.5])  # shift (1,0,0) precedes (-1,0,0), (0,1,0)
+    # near tie: |a - q|^2 = 0.25 + 2^-54 > |b - q|^2 = 0.25, but both roots round to 0.5 and the reference keeps the
+    # first of equal roots, a (voxel (0,0,0) comes first); a minimum on squared distances would answer b. The oracle's
+    # answer is checked in test_oracle_core.py::test_closest_neighbor_near_tie_is_decided_on_rounded_roots.
+    a, b = [0.5, 0.5 + 2.0**-27, 0.0], [1.0, 0.5, 0.5]
+    n = K.VoxelHashMap(1.0, 100.0, 20)
+    n.add_points(np.array([b, a]))
+    p, d = n.closest_neighbors(np.array([[0.5, 0.5, 0.5]]))
+    assert d[0] == 0.5 and np.array_equal(p[0], a)
 
 
 def test_closest_neighbors_full_size_properties(K):
@@ -210,23 +219,24 @@ def test_build_system_close(K, O, lidar, golden):
 
 
 def test_align_points_to_map_matches_oracle(K, O, lidar):
-    g, o = build_pair(K, O, lidar, 5)
-    src = O.voxel_down_sample(O.voxel_down_sample(lidar.scan(5)[0], 0.5), 1.5)
-    T5 = np.linalg.inv(lidar.pose(0)) @ lidar.pose(5)
-    reg = K.Registration(500, 1e-4, 0)
-    for tangent in ([0.3, -0.2, 0.05, 0.01, -0.01, 0.02], [0.0] * 6, [-0.5, 0.4, 0.0, 0.0, 0.0, -0.03]):
-        guess = T5 @ O.se3_exp(tangent)
-        Pg = reg.align_points_to_map(src, g, guess, 3.0, 1.0)
-        Po, it = O.align_points_to_map(o, src, guess, 3.0, 1.0)
-        dt, dr = pose_error(Pg, Po)
-        assert dt < 1e-4 and dr < 1e-4      # BASELINE bar
-        assert dt < 1e-9 and dr < 1e-9      # expected: summation-order noise only
-        assert reg.last_iterations == it
-    # max_num_iterations is honoured
-    reg1 = K.Registration(1, 1e-4, 0)
-    P1 = reg1.align_points_to_map(src, g, T5 @ O.se3_exp([0.3, 0, 0, 0, 0, 0]), 3.0, 1.0)
-    Po1, it1 = O.align_points_to_map(o, src, T5 @ O.se3_exp([0.3, 0, 0, 0, 0, 0]), 3.0, 1.0, max_iter=1)
-    assert reg1.last_iterations == 1 == it1 and np.allclose(P1, Po1, atol=1e-12)
+    for cap in (20, 37):  # 37 > 32 points per voxel: whole-grid loop, voxel-by-voxel walk
+        g, o = build_pair(K, O, lidar, 5, cap=cap)
+        src = O.voxel_down_sample(O.voxel_down_sample(lidar.scan(5)[0], 0.5), 1.5)
+        T5 = np.linalg.inv(lidar.pose(0)) @ lidar.pose(5)
+        reg = K.Registration(500, 1e-4, 0)
+        for tangent in ([0.3, -0.2, 0.05, 0.01, -0.01, 0.02], [0.0] * 6, [-0.5, 0.4, 0.0, 0.0, 0.0, -0.03]):
+            guess = T5 @ O.se3_exp(tangent)
+            Pg = reg.align_points_to_map(src, g, guess, 3.0, 1.0)
+            Po, it = O.align_points_to_map(o, src, guess, 3.0, 1.0)
+            dt, dr = pose_error(Pg, Po)
+            assert dt < 1e-4 and dr < 1e-4, (cap, dt, dr)      # BASELINE bar
+            assert dt < 1e-9 and dr < 1e-9, (cap, dt, dr)      # expected: summation-order noise only
+            assert reg.last_iterations == it, (cap, reg.last_iterations, it)
+        # max_num_iterations is honoured
+        reg1 = K.Registration(1, 1e-4, 0)
+        P1 = reg1.align_points_to_map(src, g, T5 @ O.se3_exp([0.3, 0, 0, 0, 0, 0]), 3.0, 1.0)
+        Po1, it1 = O.align_points_to_map(o, src, T5 @ O.se3_exp([0.3, 0, 0, 0, 0, 0]), 3.0, 1.0, max_iter=1)
+        assert reg1.last_iterations == 1 == it1 and np.allclose(P1, Po1, atol=1e-12), cap
 
 
 def test_align_degenerate_cases(K, O):
@@ -276,13 +286,18 @@ def test_pipeline_golden_streams(K, golden, tag):
     assert np.allclose(gp, golden[f"{tag}_map_pts"], atol=1e-9)
 
 
-@pytest.mark.parametrize("stamps,voxel", [("none", 1.0), ("column", 1.0), ("column", 0.3)])
-def test_pipeline_free_running_stream_vs_oracle(K, O, stamps, voxel):
+@pytest.mark.parametrize("stamps,voxel,cap", [
+    pytest.param("none", 1.0, 20, id="none-1.0"),
+    pytest.param("column", 1.0, 20, id="column-1.0"),
+    pytest.param("column", 0.3, 20, id="column-0.3"),
+    pytest.param("none", 1.0, 40, id="none-1.0-cap40"),  # > 32 points per voxel: no ICP team, voxel-by-voxel walk
+])
+def test_pipeline_free_running_stream_vs_oracle(K, O, stamps, voxel, cap):
     from kiss_icp_b200 import synthetic
     L = synthetic.small_shape(seed=5, beams=32, cols=512, stamps=stamps)
-    cfg = K.load_config(voxel_size=voxel)
+    cfg = K.load_config(voxel_size=voxel, mapping__max_points_per_voxel=cap)
     g = K.KissICP(cfg)
-    o = O.KissICP(voxel_size=voxel)
+    o = O.KissICP(voxel_size=voxel, max_points_per_voxel=cap)
     for k in range(25):
         p, t = L.scan(k)
         g.register_frame(p, t, return_clouds=False)

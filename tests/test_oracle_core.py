@@ -135,6 +135,19 @@ def test_closest_neighbor_is_27_neighbourhood_minimum(O):
     assert d[0] == np.finfo(float).max and np.array_equal(p[0], [0, 0, 0])
 
 
+def test_closest_neighbor_near_tie_is_decided_on_rounded_roots(O):
+    # the near tie of test_gpu_parity.py::test_closest_neighbors_golden_and_ties: |a - q|^2 = 0.25 + 2^-54 and
+    # |b - q|^2 = 0.25 differ, both roots round to 0.5, and the reference keeps the first of equal roots: a, whose voxel
+    # (0,0,0) it visits before b's (1,0,0). A minimum on squared distances would answer b.
+    a, b, q = np.array([0.5, 0.5 + 2.0**-27, 0.0]), np.array([1.0, 0.5, 0.5]), np.array([0.5, 0.5, 0.5])
+    assert ((a - q) ** 2).sum() == 0.25 + 2.0**-54 and ((b - q) ** 2).sum() == 0.25
+    assert np.sqrt(((a - q) ** 2).sum()) == np.sqrt(((b - q) ** 2).sum()) == 0.5
+    m = O.VoxelHashMap(1.0, 100.0, 20)
+    m.add_points(np.array([b, a]))
+    p, d = m.closest_neighbors(q[None], nthreads=1)
+    assert d[0] == 0.5 and np.array_equal(p[0], a)
+
+
 def test_nn_and_system_golden(O, golden):
     m = O.VoxelHashMap(1.0, 100.0, 20)
     m.add_points(golden["ds_in"])

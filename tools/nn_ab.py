@@ -28,6 +28,6 @@ for it in range(8):
     torch.cuda.synchronize()
     if it >= 3: ts.append(e0.elapsed_time(e1))
 import hashlib
-digest = hashlib.sha1(outp.cpu().numpy().tobytes() + outd.cpu().numpy().tobytes()).hexdigest()[:16]  # equal across kernel variants = bit-identical answers
-print(os.environ.get("KB_LIB", "default"), os.environ.get("KB_NN_KERNEL", "async"), "nn ms", round(float(np.median(ts)), 4), "checksum", float(outd[outd < 1e300].sum()),
+digest = hashlib.sha1(outp.cpu().numpy().tobytes() + outd.cpu().numpy().tobytes()).hexdigest()[:16]  # equal across library builds = bit-identical answers
+print(os.environ.get("KB_LIB", "default"), "nn ms", round(float(np.median(ts)), 4), "checksum", float(outd[outd < 1e300].sum()),
       "sha1(points, distances)", digest, flush=True)
